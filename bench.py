@@ -5,7 +5,11 @@ A "step" is one complete vdo_graph_optimize() call (the reference's Optimizer::F
 300 iterations, terminate action gain < 1e-4) on the config-5 factor graph, restarted from the same initial estimates
 every step; value = LM iterations executed / device time.  See DESIGN.md section "Measurement".
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config5|config4|small]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config5|config4|small] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned to its caller (se3 and pt vertex estimates, chi2 history) as
+DIR/<name>.npy in float64, all of it (44 MB on config 5).  The inputs come from a seeded generator, so two builds run with the
+same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -165,6 +169,8 @@ def run_ours(args, rank, world, local_rank):
         dist.barrier()
     clocks = sampler.stop()
     se3_fin, pt_fin = G.vertices_gathered(dist) if world > 1 else G.vertices()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, se3=se3_fin, pt=pt_fin, chi2=r["chi2"])
     parity = golden_parity(args.workload, r, se3_fin, pt_fin) if rank == 0 else None
     ms = ev0.elapsed_time(ev1)
     if world > 1:
@@ -431,6 +437,12 @@ def cpu_baseline(args, g, budget_s=20.0):
             "lm_iterations": int(r["iters"]), "seconds": dt}
 
 
+def dump_outputs(out_dir, **arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float64))
+
+
 def golden_parity(workload, r, se3, pt):
     """GPU result of the timed solve against the oracle's frozen full solve of the same config (tests/golden/ba_<workload>.npz,
     made by tests/golden/make_golden.py from the seeded generator)."""
@@ -439,7 +451,7 @@ def golden_parity(workload, r, se3, pt):
         return None
     from vdo_slam_b200.synth import iso_inv, iso_mul, iso_t, iso_R
     d = np.load(path)
-    dd = iso_mul(iso_inv(se3), d["se3"])
+    dd = iso_mul(iso_inv(se3[d["se3_idx"]] if "se3_idx" in d else se3), d["se3"])      # config 5 stores a sample of the se3 vertices
     n = min(len(r["chi2"]), len(d["chi2"]))
     return {"against": f"tests/golden/ba_{workload}.npz (oracle full solve, {int(d['iters'])} LM iterations)", "iters_equal": bool(int(d["iters"]) == int(r["iterations"])),
             "lm_iterations": int(r["iterations"]), "max_pose": float(max(np.abs(iso_t(dd)).max(), np.abs(iso_R(dd) - np.eye(3)).max())),
@@ -484,6 +496,8 @@ def run_reference(args, rank, world):
     g = make_batch_graph(**WORKLOADS[args.workload])
     w, k = max(args.warmup, 0), max(args.steps, 1)
     r = po.ba_optimize_blocked(g, max_iters=w + k, gain_threshold=0.0, nthreads=0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, se3=r["se3"], pt=r["pt"], chi2=r["chi2"])
     t = r["t_iter"]
     done = len(t)
     k_done = max(done - w, 1)
@@ -511,7 +525,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="config5", choices=[k for k in WORKLOADS if k != "cpu_sample"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
         out = run_reference(args, rank, world)

@@ -31,14 +31,19 @@ def graph_fingerprint(g):
                      float(g["ter_pph"].astype(np.int64).sum())])
 
 
-def big(name, cfg, pt_stride):
+def big(name, cfg, pt_stride, se3_stride=None):
     """Full LM solve of a BASELINE config by the oracle (blocked direct solver, oracle/ba_block.h: the same Cholesky solve of the
     full system as oracle/ba_lm.c's scalar one, which tests/test_oracle_ba.py checks on small graphs).  Keeps: iteration count,
-    chi2 / lambda history, every se3 vertex, every pt_stride-th point."""
+    chi2 / lambda history, every se3 vertex (or, with se3_stride, every se3_stride-th one, listed in se3_idx), every pt_stride-th
+    point.  The strides keep each file under 1 MB."""
     g = make_batch_graph(**cfg)
     r = po.ba_optimize_blocked(g, max_iters=300, gain_threshold=1e-4, verbose=True)
     idx = np.arange(0, len(g["pt"]), pt_stride)
-    np.savez_compressed(os.path.join(HERE, name), iters=r["iters"], chi2=r["chi2"], lam=r["lam"], se3=r["se3"], pt_idx=idx,
+    se3 = {"se3": r["se3"]}
+    if se3_stride:
+        se3_idx = np.arange(0, len(g["se3"]), se3_stride)
+        se3 = {"se3": r["se3"][se3_idx], "se3_idx": se3_idx}
+    np.savez_compressed(os.path.join(HERE, name), iters=r["iters"], chi2=r["chi2"], lam=r["lam"], **se3, pt_idx=idx,
                         pt=r["pt"][idx], fingerprint=graph_fingerprint(g), trials=r["stats"]["trials"],
                         cfg=np.array(repr(cfg)), oracle_seconds=r["stats"]["t_total"])
     print(name, "iters", r["iters"], "chi2", r["chi2"][0], "->", r["chi2"][-1], "seconds", r["stats"]["t_total"])
@@ -48,7 +53,7 @@ def main():
     if "--config4" in sys.argv:
         return big("ba_config4.npz", CONFIG4, 7)
     if "--config5" in sys.argv:
-        return big("ba_config5.npz", CONFIG5, 59)
+        return big("ba_config5.npz", CONFIG5, 177, se3_stride=4)
     # batch LM (Optimizer::FullBatchOptimization constants): 10 frames, 1 object, 120 static + 40 dynamic tracks
     g = make_batch_graph(n_frames=10, n_objects=1, n_static=120, n_dynamic=40, seed=42)
     r = po.ba_optimize(g, max_iters=12, gain_threshold=1e-4)
