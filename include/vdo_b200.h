@@ -252,6 +252,16 @@ int vdo_orb_extract(vdo_frame *f, int nfeatures, float scale_factor, int nlevels
  * non-zero flow whose target stays inside the image.  keep_idx = indices into the input, in order. */
 int vdo_frame_filter_static(vdo_frame *f, int n, const float *kx, const float *ky, float th_depth, int *keep_idx, float *cx,
                             float *cy, float *fu, float *fv, float *depth, int *n_out);
+/* Frame::SampleKeyPoints + Option II of Frame::Frame (src/Frame.cc:672-740, 130-194; UseSampleFeature: 1) on the resident images: the
+ * VDO_SAMPLE_KEYPOINTS random pixels the reference draws from cv::RNG(seed) over a 20 x 20 grid (cell-major: cell i*20+j, column cell i,
+ * row cell j; in draw order within a cell; duplicates kept), then the ones with mask == 0, 0 < depth <= th_depth, both flow components
+ * non-zero and the flow target strictly inside the image (0 < x+fu < width, 0 < y+fv < height), in that order.  kx / ky: the kept pixels
+ * (mvStatKeysTmp), cx / cy = x+fu / y+fv (mvCorres), fu / fv (mvFlowNext), depth (mvStatDepthTmp); max_out bounds these arrays.  seed 0
+ * is cv::RNG(0), i.e. the stream of seed 0xffffffff.  raw_xy (may be NULL): the VDO_SAMPLE_KEYPOINTS x 2 unfiltered samples.
+ * VDO_ERR_ARG when width or height is below 20 (the reference never leaves its sampling loop there). */
+#define VDO_SAMPLE_KEYPOINTS 3000
+int vdo_frame_sample_static(vdo_frame *f, uint32_t seed, float th_depth, int max_out, float *kx, float *ky, float *cx, float *cy, float *fu,
+                            float *fv, float *depth, int *n_out, float *raw_xy);
 /* Frame::Frame semi-dense object sampling (src/Frame.cc:200-228): raster scan with the given stride, mask != 0,
  * 0 < depth < th_depth_obj, flow target inside the image; outputs in raster (push_back) order */
 int vdo_frame_sample_objects(vdo_frame *f, float th_depth_obj, int step, int max_out, int *x, int *y, float *cx, float *cy,
@@ -362,7 +372,12 @@ typedef struct vdo_tracker_params {
   int dataset;                       /* ChooseData / mTestData (src/Tracking.cc:150-160): 1 OMD, 2 KITTI, 3 VirtualKITTI; 0 = KITTI when is_kitti else OMD.
                                         OMD and KITTI convert the raw disparity to depth (bf / (d / factor)); VirtualKITTI only clamps negatives
                                         to 0 (src/Tracking.cc:180-204) */
-  int reserved[2];
+  int use_sample_feature;            /* UseSampleFeature: 1 = background keypoints from vdo_frame_sample_static instead of the ORB keypoints
+                                        (ORB still runs: a frame without ORB keypoints stays empty, src/Frame.cc:97-98), and the RenewFrameInfo
+                                        top-up draws from that filtered sample list (src/Tracking.cc:2718-2721) */
+  unsigned sample_seed;              /* 0: every frame seeds with (unsigned)time(NULL) read when it is built, like src/Frame.cc:674; otherwise every
+                                        frame uses this seed (what the reference does for frames built within the same second).  The seed of the
+                                        last frame is vdo_tracker_get("sample_seed") */
 } vdo_tracker_params;
 void vdo_tracker_params_default(vdo_tracker_params *p);
 int vdo_tracker_create(vdo_ctx *ctx, const vdo_tracker_params *params, vdo_tracker **out);
@@ -382,7 +397,8 @@ int vdo_tracker_track(vdo_tracker *t, int width, int height, const unsigned char
  * mvObjCorres mvObjFlowNext mvObj3DPoint vSemObjLabel vObjLabel nDynInlierID vFlow_3d nModLabel nSemPosition bObjStat vObjMod
  * vObjCentre3D TemperalMatch_subset max_id f_id; stage_ms (9 x f32, accumulated host wall-clock per stage since creation: upload+depth, mask,
  * frame build (ORB + static filter + object samples), look-ups, initial camera model, camera LM, objects, renewal, windowed BA);
- * local_ba (2 x i32: windowed optimisations run, their LM iterations) */
+ * local_ba (2 x i32: windowed optimisations run, their LM iterations); sample_seed (1 x u32: the seed the last frame sampled with, 0 when it did
+ * not sample) */
 int vdo_tracker_get(const vdo_tracker *t, const char *name, void *out, int cap_elems, int *n_elems);
 
 /* Map -> factor graph -> optimise -> write back (SURVEY.md 8f N2): mode 0 = Optimizer::PartialBatchOptimization(pMap, K, WINDOW_SIZE)

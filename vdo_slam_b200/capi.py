@@ -395,6 +395,20 @@ class Frame:
         k = m.value
         return (idx[:k],) + tuple(a[:k] for a in out)
 
+    SAMPLE_KEYPOINTS = 3000      # VDO_SAMPLE_KEYPOINTS
+
+    def sample_static(self, seed, th_depth):
+        """vdo_frame_sample_static: Frame::SampleKeyPoints (cv::RNG(seed); seed 0 = stream of 0xffffffff) + the Option II filter.
+        Returns dict(raw (3000, 2) unfiltered samples, x, y, cx, cy, fu, fv, depth of the kept ones, in order)."""
+        n = self.SAMPLE_KEYPOINTS
+        out = [np.zeros(n, np.float32) for _ in range(7)]
+        raw = np.zeros((n, 2), np.float32)
+        m = C.c_int(0)
+        self.ctx.check(self.ctx.L.vdo_frame_sample_static(self.h_, C.c_uint32(seed), C.c_float(th_depth), C.c_int(n), *[_fp(a) for a in out], C.byref(m), _fp(raw)),
+                       "vdo_frame_sample_static")
+        k = m.value
+        return dict(raw=raw, **{name: a[:k] for name, a in zip(("x", "y", "cx", "cy", "fu", "fv", "depth"), out)})
+
     def sample_objects(self, th_depth_obj, step=4, max_out=None):
         max_out = max_out or ((self.w + step - 1) // step) * ((self.h + step - 1) // step)
         x, y, lab = (np.zeros(max_out, np.int32) for _ in range(3))
@@ -565,12 +579,14 @@ class TrackerParams(C.Structure):
                 ("depth_factor", C.c_float), ("th_depth_bg", C.c_float), ("th_depth_obj", C.c_float), ("max_track_bg", C.c_int), ("max_track_obj", C.c_int),
                 ("sf_mg_thres", C.c_float), ("sf_ds_thres", C.c_float), ("n_features", C.c_int), ("scale_factor", C.c_float), ("n_levels", C.c_int),
                 ("ini_th_fast", C.c_int), ("min_th_fast", C.c_int), ("is_kitti", C.c_int), ("quirk", C.c_int), ("window_size", C.c_int),
-                ("overlap_size", C.c_int), ("local_batch", C.c_int), ("dataset", C.c_int), ("reserved", C.c_int * 2)]
+                ("overlap_size", C.c_int), ("local_batch", C.c_int), ("dataset", C.c_int), ("use_sample_feature", C.c_int),
+                ("sample_seed", C.c_uint)]
 
 
 class Tracker:
     """vdo_tracker: System::TrackRGBD -> Tracking::GrabImageRGBD -> Tracking::Track on the device stages."""
-    _INT = {"nStaInlierID", "vSemObjLabel", "vObjLabel", "nDynInlierID", "nModLabel", "nSemPosition", "bObjStat", "TemperalMatch_subset", "max_id", "f_id", "local_ba"}
+    _INT = {"nStaInlierID", "vSemObjLabel", "vObjLabel", "nDynInlierID", "nModLabel", "nSemPosition", "bObjStat", "TemperalMatch_subset", "max_id", "f_id", "local_ba",
+            "sample_seed"}
 
     def __init__(self, ctx: Context, **overrides):
         self.ctx = ctx

@@ -9,6 +9,8 @@
 //                               against cv2 4.13 in tests/test_image_oracle.py
 //   Frame static filter         src/Frame.cc:100-129, 181-194
 //   Frame object sampling       src/Frame.cc:200-228
+//   sampled background keys     src/Frame.cc:672-740 (SampleKeyPoints, cv::RNG), 130-194 (Option II filter); restated in
+//                               oracle/sampled_features.py
 //   back-projection, scene flow src/Frame.cc:484-555, src/Tracking.cc:1278-1364
 //
 // A KITTI frame is 1242x375 (0.47 Mpx, ~9 MB of inputs): every kernel here is launch-/latency-bound, not HBM-bound; the
@@ -310,6 +312,97 @@ __global__ void __launch_bounds__(1024) k_filter_static(const float* __restrict_
   if (threadIdx.x == 0) *n_out = base;
 }
 
+// ------------------------------------------------------------------------------------------------ sampled background keypoints
+// Frame::SampleKeyPoints (src/Frame.cc:672-740) + Option II of the Frame constructor (:130-194).  cv::RNG is multiply-with-carry,
+// s <- (s mod 2^32) * A + floor(s / 2^32), returning (uint32)s.  That step is s * r mod m with m = A * 2^32 - 1 and r = 2^-32 mod m
+// (A * 2^32 == 1 mod m), so the state after k draws is seed * r^k mod m and every draw is independent of the others given a table
+// of powers of r.  The reference's loop visits cell c = v % 400 at visit v (column cell i = c / 20 outer, row cell j = c % 20 inner)
+// and draws x then y, i.e. draws 2v+1 and 2v+2.  Only the 39 cells with i == 0 or j == 0 can reject a visit, so 3 000 samples
+// need at most 9 sweeps of 400 visits.
+constexpr unsigned long long RNG_A = 4164903690ull, RNG_M = 0xf83f6309ffffffffull;
+constexpr int SAMP_DIV = 20, SAMP_CELLS = SAMP_DIV * SAMP_DIV, SAMP_SWEEPS = 9, SAMP_VISITS = SAMP_CELLS * SAMP_SWEEPS, SAMP_DRAWS = 2 * SAMP_VISITS;
+static_assert(VDO_SAMPLE_KEYPOINTS <= (SAMP_CELLS - 2 * SAMP_DIV + 1) * SAMP_SWEEPS, "9 sweeps must always yield the samples");
+
+// (uint32)(seed * t * r^2 mod m) for seed < 2^32, t < m: two MWC steps on the 96-bit product (each multiplies by r), then one
+// conditional subtraction (the second step leaves a value below m + 2^33 < 2m)
+__device__ __forceinline__ unsigned rng_draw(unsigned seed, unsigned long long t) {
+  const unsigned long long lo = (unsigned long long)seed * t, hi = __umul64hi((unsigned long long)seed, t);
+  const unsigned long long a = (lo & 0xffffffffull) * RNG_A, s = a + ((hi << 32) | (lo >> 32));
+  const unsigned long long carry = s < a;                                   // the first step can reach 2^65
+  unsigned long long s2 = (s & 0xffffffffull) * RNG_A + ((carry << 32) | (s >> 32));
+  if (s2 >= RNG_M) s2 -= RNG_M;
+  return (unsigned)s2;
+}
+struct SampOut { float kx, ky, cx, cy, fu, fv, depth; };
+// One CTA: the 3 000 kept visits depend on a prefix count over all visits, and their cell-major placement on counts over all cells.
+// rpow[k] = r^(k-1) mod m, so draw k (1-based) is rng_draw(seed, rpow[k - 1]).
+__global__ void __launch_bounds__(1024) k_sample_static(const unsigned long long* __restrict__ rpow, unsigned seed, const int* __restrict__ mask,
+                                                         const float* __restrict__ depth, const float* __restrict__ flow, int w, int h, float th,
+                                                         float* __restrict__ raw, SampOut* __restrict__ out, int* __restrict__ n_out) {
+  __shared__ int vx[SAMP_VISITS], vy[SAMP_VISITS];
+  __shared__ unsigned char keep[SAMP_VISITS];
+  __shared__ short ord[VDO_SAMPLE_KEYPOINTS];           // visit of each output slot, cell-major
+  __shared__ int wsum[33];
+  const int xs = w / SAMP_DIV, ys = h / SAMP_DIV;
+  // (1) draws and acceptance; the loop's `break` keeps the first VDO_SAMPLE_KEYPOINTS accepted visits
+  int base = 0;
+  for (int start = 0; start < SAMP_VISITS; start += blockDim.x) {
+    const int v = start + threadIdx.x;
+    int ok = 0;
+    if (v < SAMP_VISITS) {
+      const int c = v % SAMP_CELLS, i = c / SAMP_DIV, j = c % SAMP_DIV;
+      const int x = i * xs + (int)(rng_draw(seed, rpow[2 * v]) % (unsigned)xs);        // rng.uniform(i*x_step, (i+1)*x_step)
+      const int y = j * ys + (int)(rng_draw(seed, rpow[2 * v + 1]) % (unsigned)ys);
+      ok = !(x >= w || y >= h || x <= 0 || y <= 0);
+      vx[v] = x; vy[v] = y;
+    }
+    int tot;
+    const int rank = base + cta_excl_scan(ok, wsum, tot);
+    if (v < SAMP_VISITS) keep[v] = ok && rank < VDO_SAMPLE_KEYPOINTS;
+    base += tot;
+    __syncthreads();
+  }
+  // (2) cell-major placement (KeyinGrid[i*20+j] in draw order): slot = kept visits of the earlier cells + rank within the own cell
+  int cnt = 0;
+  if (threadIdx.x < SAMP_CELLS)
+    for (int q = 0; q < SAMP_SWEEPS; ++q) cnt += keep[threadIdx.x + q * SAMP_CELLS];
+  int n_raw;
+  int pos = cta_excl_scan(cnt, wsum, n_raw);
+  if (threadIdx.x < SAMP_CELLS)
+    for (int q = 0; q < SAMP_SWEEPS; ++q) {
+      const int v = threadIdx.x + q * SAMP_CELLS;
+      if (keep[v]) ord[pos++] = (short)v;
+    }
+  __syncthreads();
+  if (raw)
+    for (int k = threadIdx.x; k < n_raw; k += blockDim.x) { raw[2 * k] = (float)vx[ord[k]]; raw[2 * k + 1] = (float)vy[ord[k]]; }
+  // (3) Option II filter, ordered compaction
+  base = 0;
+  for (int start = 0; start < n_raw; start += blockDim.x) {
+    const int k = start + threadIdx.x;
+    int ok = 0; float px = 0, py = 0, fx = 0, fy = 0, tx = 0, ty = 0, d = 0;
+    if (k < n_raw) {
+      const int x = vx[ord[k]], y = vy[ord[k]];
+      px = (float)x; py = (float)y;
+      const size_t p = (size_t)y * w + x;
+      d = depth[p];
+      if (mask[p] == 0 && !(d > th || d <= 0.f)) {
+        fx = flow[2 * p]; fy = flow[2 * p + 1];
+        if (fx != 0.f && fy != 0.f) {
+          tx = __fadd_rn(px, fx); ty = __fadd_rn(py, fy);
+          ok = (tx < (float)w && ty < (float)h && tx > 0.f && ty > 0.f);
+        }
+      }
+    }
+    int tot;
+    const int o = base + cta_excl_scan(ok, wsum, tot);
+    if (ok) out[o] = SampOut{px, py, tx, ty, fx, fy, d > 0.f ? d : -1.f};
+    base += tot;
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) *n_out = base;
+}
+
 // Dense packing of the per-cell candidate lists (cell-major, row-major inside a cell = the order the host octree expects):
 // k_cell_offsets: exclusive scan of the cell counts by one CTA; k_cell_gather: one CTA per cell copies its entries.
 // Only count + offsets (a few KB) and the packed candidates (~0.3 MB) cross PCIe instead of ncell * CELL_CAP slots (~8 MB).
@@ -549,6 +642,7 @@ struct vdo_frame {
   KpLvl* kps = nullptr; float* ang = nullptr; int kp_cap = 0, n_kps = -1;    // keypoints (level coordinates) / angles of the last vdo_orb_extract
   unsigned char* blur[MAX_LEVELS] = {nullptr};
   void* scratch = nullptr; size_t scratch_cap = 0; int* d_count = nullptr;
+  unsigned long long* samp_pow = nullptr;        // r^(k-1) mod m for the SAMP_DRAWS draws of vdo_frame_sample_static (seed-independent)
   std::vector<KpOut> h_cell_out; std::vector<int> h_cell_cnt;
   OrbSetup orb; bool orb_ready = false;
   int launches = 0;
@@ -578,7 +672,7 @@ extern "C" void vdo_frame_destroy(vdo_frame* f) {
   for (int l = 1; l < MAX_LEVELS; ++l) cudaFree(f->pyr[l]);
   for (int l = 0; l < MAX_LEVELS; ++l) { cudaFree(f->score[l]); cudaFree(f->blur[l]); }
   cudaFree(f->cells); cudaFree(f->cell_out); cudaFree(f->cell_cnt); cudaFree(f->kps); cudaFree(f->ang); cudaFree(f->scratch);
-  cudaFree(f->cell_off); cudaFree(f->cell_dense); cudaFreeHost(f->h_cnt_off); cudaFreeHost(f->h_dense);
+  cudaFree(f->cell_off); cudaFree(f->cell_dense); cudaFreeHost(f->h_cnt_off); cudaFreeHost(f->h_dense); cudaFree(f->samp_pow);
   delete f;
 }
 // D2H of the resident mask (the tracker writes it back into the caller's buffer only when UpdateMask changed it)
@@ -782,6 +876,35 @@ extern "C" int vdo_frame_filter_static(vdo_frame* f, int n, const float* kx, con
   std::vector<StatOut> h(m);
   if (m) { FRK(cudaMemcpyAsync(h.data(), d_out, sizeof(StatOut) * m, cudaMemcpyDeviceToHost, f->st)); FRK(cudaStreamSynchronize(f->st)); }
   for (int i = 0; i < m; ++i) { keep_idx[i] = h[i].idx; cx[i] = h[i].cx; cy[i] = h[i].cy; fu[i] = h[i].fu; fv[i] = h[i].fv; depth[i] = h[i].depth; }
+  *n_out = m;
+  return VDO_OK;
+}
+
+extern "C" int vdo_frame_sample_static(vdo_frame* f, uint32_t seed, float th_depth, int max_out, float* kx, float* ky, float* cx, float* cy, float* fu,
+                                       float* fv, float* depth, int* n_out, float* raw_xy) {
+  if (!f || max_out < 0 || !n_out || (max_out && (!kx || !ky || !cx || !cy || !fu || !fv || !depth))) return VDO_ERR_ARG;
+  if (f->w < SAMP_DIV || f->h < SAMP_DIV) return VDO_ERR_ARG;         // an empty grid step: the reference's loop never ends
+  if (!f->samp_pow) {
+    std::vector<unsigned long long> tab(SAMP_DRAWS);
+    unsigned long long s = 1ull << 32;                                  // r^-1 mod m; one MWC step multiplies by r
+    for (int k = 0; k < SAMP_DRAWS; ++k) { tab[k] = s; s = (s & 0xffffffffull) * RNG_A + (s >> 32); }
+    FRK(cudaMalloc(&f->samp_pow, sizeof(unsigned long long) * SAMP_DRAWS));
+    FRK(cudaMemcpyAsync(f->samp_pow, tab.data(), sizeof(unsigned long long) * SAMP_DRAWS, cudaMemcpyHostToDevice, f->st));
+    FRK(cudaStreamSynchronize(f->st));
+  }
+  const int N = VDO_SAMPLE_KEYPOINTS;
+  if (int rc = ensure_scratch(f, sizeof(float) * 2 * N + sizeof(SampOut) * N + 64)) return rc;
+  float* d_raw = (float*)f->scratch; SampOut* d_out = (SampOut*)(d_raw + 2 * N);
+  k_sample_static<<<1, 1024, 0, f->st>>>(f->samp_pow, seed ? seed : 0xffffffffu, f->mask, f->depth, f->flow, f->w, f->h, th_depth, raw_xy ? d_raw : nullptr, d_out,
+                                         f->d_count); f->launches++;
+  int m = 0;
+  FRK(cudaMemcpyAsync(&m, f->d_count, sizeof(int), cudaMemcpyDeviceToHost, f->st));
+  if (raw_xy) FRK(cudaMemcpyAsync(raw_xy, d_raw, sizeof(float) * 2 * N, cudaMemcpyDeviceToHost, f->st));
+  FRK(cudaStreamSynchronize(f->st));
+  m = std::min(m, max_out);
+  std::vector<SampOut> h(m);
+  if (m) { FRK(cudaMemcpyAsync(h.data(), d_out, sizeof(SampOut) * m, cudaMemcpyDeviceToHost, f->st)); FRK(cudaStreamSynchronize(f->st)); }
+  for (int i = 0; i < m; ++i) { kx[i] = h[i].kx; ky[i] = h[i].ky; cx[i] = h[i].cx; cy[i] = h[i].cy; fu[i] = h[i].fu; fv[i] = h[i].fv; depth[i] = h[i].depth; }
   *n_out = m;
   return VDO_OK;
 }

@@ -12,6 +12,7 @@
 #include <cstdlib>
 #include <chrono>
 #include <cstring>
+#include <ctime>
 #include <string>
 #include <vector>
 
@@ -54,6 +55,7 @@ struct FrameState {
   std::vector<float> keys;                                              // mvKeys (x, y)
   std::vector<float> statKeysTmp, corres, flowNext, statDepthTmp, stat3DTmp;   // mvStatKeysTmp, mvCorres, mvFlowNext, mvStatDepthTmp, mvStat3DPointTmp
   std::vector<float> statKeys, statDepth;                               // mvStatKeys, mvStatDepth
+  std::vector<float> sampKeys;                                          // Option II: the constructor's filtered samples (RenewFrameInfo's top-up source)
   std::vector<int> staInlierID;                                         // nStaInlierID
   std::vector<float> objKeys, objCorres, objFlowNext, objDepth, obj3D;  // mvObjKeys, mvObjCorres, mvObjFlowNext, mvObjDepth, mvObj3DPoint
   std::vector<int> semObjLabel, objLabel, dynInlierID;                  // vSemObjLabel, vObjLabel, nDynInlierID
@@ -64,7 +66,7 @@ struct FrameState {
   std::vector<float> vObjCentre3D;                                      // 3 per object (src/Tracking.cc:856-866)
   std::vector<std::vector<int>> vnObjID, vnObjInlierID;
   void clear_dynamic() {
-    keys.clear(); statKeysTmp.clear(); corres.clear(); flowNext.clear(); statDepthTmp.clear(); stat3DTmp.clear(); statKeys.clear(); statDepth.clear();
+    keys.clear(); statKeysTmp.clear(); corres.clear(); flowNext.clear(); statDepthTmp.clear(); stat3DTmp.clear(); statKeys.clear(); statDepth.clear(); sampKeys.clear();
     staInlierID.clear(); objKeys.clear(); objCorres.clear(); objFlowNext.clear(); objDepth.clear(); obj3D.clear(); semObjLabel.clear(); objLabel.clear();
     dynInlierID.clear(); flow3d.clear(); nModLabel.clear(); nSemPosition.clear(); semPosiGt.clear(); bObjStat.clear(); vObjMod.clear(); vObjCentre3D.clear(); vnObjID.clear();
     vnObjInlierID.clear();
@@ -95,6 +97,7 @@ struct vdo_tracker {
   std::string err;
   double stage_ms[9] = {0};
   int frames = 0, local_ba_runs = 0, local_ba_iters = 0;
+  unsigned sample_seed = 0;    // seed of the last frame's sampled background keypoints (0: none drawn)
   // scratch
   std::vector<float> s_f[12]; std::vector<int> s_i[8]; std::vector<unsigned char> s_b[2]; std::vector<double> s_d[2];
 };
@@ -133,16 +136,27 @@ int build_frame(vdo_tracker* t, FrameState& F) {
   F.keys.resize(2 * (size_t)n);
   for (int i = 0; i < n; ++i) { F.keys[2 * i] = x[i]; F.keys[2 * i + 1] = y[i]; }
   if (n == 0) return VDO_OK;                                    // Frame.cc:83-84: nothing else is filled
+  const bool sampled = p.use_sample_feature != 0;
+  const int ns = sampled ? VDO_SAMPLE_KEYPOINTS : n;
   auto& keep = t->s_i[2]; auto& cx = t->s_f[4]; auto& cy = t->s_f[5]; auto& fu = t->s_f[6]; auto& fv = t->s_f[7]; auto& dp = t->s_f[8];
-  keep.resize(n); cx.resize(n); cy.resize(n); fu.resize(n); fv.resize(n); dp.resize(n);
+  keep.resize(ns); cx.resize(ns); cy.resize(ns); fu.resize(ns); fv.resize(ns); dp.resize(ns);
   int m = 0;
-  TK(vdo_frame_filter_static(F.img, n, x.data(), y.data(), p.th_depth_bg, keep.data(), cx.data(), cy.data(), fu.data(), fv.data(), dp.data(), &m));
+  if (sampled) {                                                // Option II (Frame.cc:130-194)
+    const unsigned seed = p.sample_seed ? p.sample_seed : (unsigned)std::time(nullptr);   // cv::RNG rng((unsigned)time(NULL)), Frame.cc:674
+    t->sample_seed = seed;
+    x.resize(ns); y.resize(ns);                                 // the ORB keypoints are in F.keys already
+    TK(vdo_frame_sample_static(F.img, seed, p.th_depth_bg, ns, x.data(), y.data(), cx.data(), cy.data(), fu.data(), fv.data(), dp.data(), &m, nullptr));
+    for (int i = 0; i < m; ++i) keep[i] = i;
+  } else {
+    TK(vdo_frame_filter_static(F.img, n, x.data(), y.data(), p.th_depth_bg, keep.data(), cx.data(), cy.data(), fu.data(), fv.data(), dp.data(), &m));
+  }
   F.statKeysTmp.resize(2 * (size_t)m); F.corres.resize(2 * (size_t)m); F.flowNext.resize(2 * (size_t)m); F.statDepthTmp.resize(m);
   for (int i = 0; i < m; ++i) {
     F.statKeysTmp[2 * i] = x[keep[i]]; F.statKeysTmp[2 * i + 1] = y[keep[i]];
     F.corres[2 * i] = cx[i]; F.corres[2 * i + 1] = cy[i]; F.flowNext[2 * i] = fu[i]; F.flowNext[2 * i + 1] = fv[i];
     F.statDepthTmp[i] = dp[i] > 0 ? dp[i] : -1.f;
   }
+  if (sampled) F.sampKeys = F.statKeysTmp;                     // RenewFrameInfo overwrites mvStatKeysTmp but tops up from this list
   const int step = 4, cap = ((p.width + step - 1) / step) * ((p.height + step - 1) / step);
   auto& ox = t->s_i[3]; auto& oy = t->s_i[4]; auto& lab = t->s_i[5];
   auto& ocx = t->s_f[4]; auto& ocy = t->s_f[5]; auto& ofx = t->s_f[6]; auto& ofy = t->s_f[7]; auto& od = t->s_f[8];
@@ -327,14 +341,15 @@ int track_frame(vdo_tracker* t, FrameState& C, FrameState& L) {
     const M4 Twc = inv4(C.Tcw);
     std::vector<int> ib(nobj + 1, 0), ii;
     for (int i = 0; i < nobj; ++i) { ii.insert(ii.end(), C.vnObjInlierID[i].begin(), C.vnObjInlierID[i].end()); ib[i + 1] = (int)ii.size(); }
-    const int nTm = (int)t->temperalMatchSubset.size(), nSamp = (int)C.keys.size() / 2, nTmp = (int)t->tmpSemObjLabel.size();
+    const std::vector<float>& samp = p.use_sample_feature ? C.sampKeys : C.keys;     // mvKeysSample (:2716-2721)
+    const int nTm = (int)t->temperalMatchSubset.size(), nSamp = (int)samp.size() / 2, nTmp = (int)t->tmpSemObjLabel.size();
     const int capS = nTm + nSamp + 8, capO = (int)ii.size() + (nobj + 1) * nTmp + 8;
     std::vector<float> sk(2 * (size_t)capS), sc(2 * (size_t)capS), sf(2 * (size_t)capS), sd(capS), s3(3 * (size_t)capS);
     std::vector<int> sid(capS);
     std::vector<float> okk(2 * (size_t)capO), od(capO), oc(2 * (size_t)capO), of(2 * (size_t)capO), o3(3 * (size_t)capO);
     std::vector<int> osem(capO), oid(capO), olab(capO);
     int ns = 0, no = 0;
-    TK(vdo_renew_frame_info(C.img, nTm, t->temperalMatchSubset.data(), Ns, C.statKeys.data(), nSamp, C.keys.data(), p.max_track_bg, nobj, ib.data(), ii.data(),
+    TK(vdo_renew_frame_info(C.img, nTm, t->temperalMatchSubset.data(), Ns, C.statKeys.data(), nSamp, samp.data(), p.max_track_bg, nobj, ib.data(), ii.data(),
                             C.bObjStat.data(), C.nSemPosition.data(), C.nModLabel.data(), No, C.objKeys.data(), C.objLabel.data(), nTmp, t->tmpObjKeys.data(),
                             t->tmpObjDepth.data(), t->tmpSemObjLabel.data(), t->tmpObjFlowNext.data(), t->tmpObjCorres.data(), p.max_track_obj, K4, Twc.data(), capS, &ns,
                             sk.data(), sc.data(), sf.data(), sid.data(), sd.data(), s3.data(), capO, &no, okk.data(), od.data(), oc.data(), of.data(), osem.data(),
@@ -446,6 +461,7 @@ extern "C" int vdo_tracker_track(vdo_tracker* t, int width, int height, const un
   vdo_frame* img = C.img;
   C.clear_dynamic(); C.img = img; C.Tcw = eye4();
   if (t->first) t->f_id = 0;
+  t->sample_seed = 0;
   {
     StageTimer stage_timer_0(&t->stage_ms[0]);
     TK(vdo_frame_upload(C.img, gray, depth, flow, mask));
@@ -520,7 +536,7 @@ extern "C" int vdo_tracker_track(vdo_tracker* t, int width, int height, const un
 // Named read-back of the state after the last vdo_tracker_track call (parity tests, host shim).  kind: 'f' float, 'i' int.
 // Names: Tcw, mvKeys, mvStatKeys(Tmp), mvStatDepth(Tmp), mvCorres, mvFlowNext, mvStat3DPointTmp, nStaInlierID, mvObjKeys, mvObjDepth, mvObjCorres,
 // mvObjFlowNext, mvObj3DPoint, vSemObjLabel, vObjLabel, nDynInlierID, vFlow_3d, nModLabel, nSemPosition, bObjStat, vObjMod, TemperalMatch_subset,
-// max_id, f_id, mVelocity
+// max_id, f_id, mVelocity, sample_seed
 extern "C" int vdo_tracker_get(const vdo_tracker* t, const char* name, void* out, int cap_elems, int* n_elems) {
   if (!t || !name || !n_elems) return VDO_ERR_ARG;
   const FrameState& C = t->fr[t->cur];
@@ -555,6 +571,7 @@ extern "C" int vdo_tracker_get(const vdo_tracker* t, const char* name, void* out
   if (s == "f_id") return put_i(&t->f_id, 1);
   if (s == "stage_ms") { float v[9]; for (int i = 0; i < 9; ++i) v[i] = (float)t->stage_ms[i]; return put_f(v, 9); }
   if (s == "local_ba") { const int v[2] = {t->local_ba_runs, t->local_ba_iters}; return put_i(v, 2); }
+  if (s == "sample_seed") return put_i(reinterpret_cast<const int*>(&t->sample_seed), 1);
   return VDO_ERR_ARG;
 }
 

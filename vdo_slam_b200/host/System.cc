@@ -139,10 +139,20 @@ System::System(const string &strSettingsFile, const eSensor sensor) : mSensor(se
   p.window_size = (int)get(kv, "WINDOW_SIZE"); p.overlap_size = (int)get(kv, "OVERLAP_SIZE");
   mbRGB = (int)get(kv, "Camera.RGB") != 0;
   mbKitti = p.is_kitti != 0;
-  if ((int)get(kv, "UseSampleFeature") == 1) {
-    cerr << "UseSampleFeature: 1 draws its samples from cv::RNG(time(NULL)) in the reference and is not reproducible; not supported." << endl;
+  const int useSample = (int)get(kv, "UseSampleFeature");
+  if (useSample != 0 && useSample != 1) {
+    cerr << "UseSampleFeature must be 0 (detected features) or 1 (sampled features); got " << useSample << endl;
     exit(-1);
   }
+  p.use_sample_feature = useSample;
+  // SampleSeed is not a key of the reference: missing or 0 seeds every frame's sampler with time(NULL) like src/Frame.cc:674; any other value
+  // fixes the seed so that a run can be repeated (the tracker reports the seeds it used through vdo_tracker_get("sample_seed"))
+  const double seed = get(kv, "SampleSeed");
+  if (!(seed >= 0.0 && seed <= 4294967295.0) || seed != floor(seed)) {
+    cerr << "SampleSeed must be an integer in [0, 4294967295]; got " << seed << endl;
+    exit(-1);
+  }
+  p.sample_seed = (unsigned)seed;
   if (vdo_ctx_create(0, &mpCtx) != VDO_OK) {
     cerr << "vdo_b200: no usable CUDA device (there is no CPU fallback)" << endl;
     exit(-1);

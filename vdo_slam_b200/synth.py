@@ -299,9 +299,9 @@ def _cam_pose(t, speed=0.8, yaw_rate=0.002):
     return T
 
 
-def make_sequence_frame(t, seed=0, width=1242, height=375, n_obj=3, flow_sigma=0.2, K=None, cam_h=1.65, half_w=7.0):
-    """Frame t of the sequence `seed`.  Returns dict(gray, depth_raw (disparity*256, f32), flow (H,W,2 to frame t+1), mask,
-    Twc (4x4 f64 ground truth), obj_ids (semantic ids visible), K)."""
+def make_sequence_frame(t, seed=0, width=1242, height=375, n_obj=3, flow_sigma=0.2, K=None, cam_h=1.65, half_w=7.0, depth_factor=KITTI_DEPTH_FACTOR):
+    """Frame t of the sequence `seed`.  Returns dict(gray, depth_raw (disparity*depth_factor, f32: 256 = KITTI's DepthMapFactor, 1000 =
+    OMD's), flow (H,W,2 to frame t+1), mask, Twc (4x4 f64 ground truth), obj_ids (semantic ids visible), K)."""
     K = KITTI_K if K is None else K
     fx, fy, cx, cy = [float(v) for v in K]
     rng_o = np.random.default_rng(1000 + seed)
@@ -339,7 +339,7 @@ def make_sequence_frame(t, seed=0, width=1242, height=375, n_obj=3, flow_sigma=0
     flow = np.stack([u1 - uu, v1 - vv], -1) + rng.normal(0, flow_sigma, uu.shape + (2,))
     flow = flow.astype(np.float32)
     flow[rng.random(uu.shape) < 0.005] = 0.0
-    disp = np.round(KITTI_BF * KITTI_DEPTH_FACTOR / np.maximum(z, 0.5))
+    disp = np.round(KITTI_BF * np.float32(depth_factor) / np.maximum(z, 0.5))
     depth_raw = disp.astype(np.float32)
     depth_raw[rng.random(uu.shape) < 0.005] = -1.0
     gray = make_frame(seed=31 * seed + t, width=width, height=height, n_obj=0)["gray"]
